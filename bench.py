@@ -3,6 +3,12 @@
 
   python bench.py --gpus N --steps K --warmup W            (N>1: launched by torch.distributed.run, one rank per GPU)
   python bench.py --impl reference ...                      (the CPU arm: the oracle port on the host cores)
+  python bench.py ... --dump-outputs DIR                    (also writes what the last timed step computed, DIR/<name>.npy)
+
+Every timed loop of training steps (`e2e`, `value`, the step without the engine in `roofline`, the CPU arm) runs exactly K
+steps.  Inputs, initial variables and per-step noise are seeded.  With --dump-outputs the last timed step starts from the
+initial variables and optimizer state (restored outside the timed window), so what it computes depends on the arguments
+alone and two runs, or two builds, can be compared output for output.
 
 A "step" is one full optimisation step of --config (default cfg2 = configs[1] of BASELINE.json: SAVP, bair_action_free/ours_savp
 hparams: VAE+GAN, 64x64x3, 2 context + 10 predicted, batch 16 per GPU): generator forward (posterior + prior unrolls),
@@ -22,6 +28,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -164,7 +171,7 @@ def run_reference(args):
         return
     sample_b = cpu_sample_batch()
     S = SAVP_HPARAMS['sequence_length'] - 1
-    k = max(3, min(args.steps, 5))
+    k = args.steps
     times, cores = oracle_step_time(sample_b, k)
     med = sorted(times)[len(times) // 2]
     fps = sample_b * S / med
@@ -297,6 +304,29 @@ def engine_profile(model, batch):
             os.environ['VP_CONCURRENT_D'] = old
 
 
+DUMP_CAP = 1 << 22     # elements per dumped array (16 MB of float32): at most two arrays reach it, so a dump stays < 64 MB
+
+
+def dump_outputs(model, losses, out_dir):
+    """Writes what the last timed step computed, as a caller of train_step() + losses() receives it, to out_dir/<name>.npy:
+    every loss term (float64 scalars) and the step's generated frames and posterior statistics (float32, batch-major as
+    `model.outputs` holds them).  An array of more than DUMP_CAP
+    elements is written as <name>_sample.npy: its flattened elements at DUMP_CAP positions drawn with a fixed seed, in
+    ascending order."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in losses.items():
+        np.save(os.path.join(out_dir, k + '.npy'), np.float64(v))
+    keys = ('gen_images', 'gen_images_enc', 'zs_mu_enc', 'zs_log_sigma_sq_enc') if model.hparams.nz else ('gen_images',)
+    arrays = {k: model.outputs_time_major(k).transpose(0, 1) for k in keys}
+    for name, v in arrays.items():
+        if v.numel() > DUMP_CAP:
+            idx = np.sort(np.random.default_rng(0).choice(v.numel(), DUMP_CAP, replace=False))
+            v, name = v.reshape(-1)[torch.from_numpy(idx).to(v.device)], name + '_sample'
+        np.save(os.path.join(out_dir, name + '.npy'), v.detach().float().contiguous().cpu().numpy())
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -314,6 +344,12 @@ def run_ours(args):
     log('building model %s (batch %d per GPU)' % (args.config, B))
     model.build_graph(batch0)
     assert model.world_size == world
+    initial = None
+    if args.dump_outputs:
+        # every step adds summation-order noise (atomics) that Adam and the GAN game amplify (two runs end ~30 % apart after
+        # 50 steps), so the last timed step of a dump run starts again from these seeded initial variables and optimizer state
+        initial = tempfile.TemporaryDirectory()
+        model.save(initial.name)
     log('built; warming up the eager path')
     S = model.S
     frames_per_step = world * B * S
@@ -330,7 +366,7 @@ def run_ours(args):
     if world > 1:
         dist.barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    k_e2e = max(3, min(args.steps, 10))
+    k_e2e = args.steps
     t0 = time.time()
     e0.record()
     for i in range(k_e2e):
@@ -366,14 +402,28 @@ def run_ours(args):
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0, e1, e2, e3 = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
     torch.cuda.synchronize()
     e0.record()
-    for _ in range(args.steps):
+    for _ in range(args.steps - (initial is not None)):
         one_step()
     e1.record()
+    if initial is not None:
+        # the last timed step of a dump run starts from the seeded initial state, restored outside the timed window; its
+        # host-side staging runs before its start event too, as it does under the GPU work of the step before in the loop
+        model.restore(None, initial.name)     # copies into the buffers the captured graph reads
+        initial.cleanup()
+        model.redraw_step_randomness()
+        model.stage_step()
+        e2.record()
+        if graph is not None:
+            graph.replay()                    # what one_step() runs after the same staging
+        else:
+            model._step_device(getattr(model, '_allreduce', None))
+        model.global_step += 1
+        e3.record()
     torch.cuda.synchronize()
-    ms = e0.elapsed_time(e1) / args.steps
+    ms = (e0.elapsed_time(e1) + (e2.elapsed_time(e3) if initial is not None else 0.0)) / args.steps
     sampler.stop_flag = True
     log('%.2f ms/step' % ms)
     if world > 1:
@@ -383,11 +433,14 @@ def run_ours(args):
         dist.barrier()
     losses = model.losses()
     finite = all(v == v for v in losses.values())
+    if args.dump_outputs and rank == 0:      # before the roofline legs, which run steps whose results are garbage by design
+        dump_outputs(model, losses, args.dump_outputs)
+        log('outputs of the last timed step written to %s' % args.dump_outputs)
 
     # ---------------- rooflines + CPU baseline (rank 0; the CPU leg at N = 1 only)
     no_engine_ms = None
     if not args.no_roofline and world == 1 and graph is not None:
-        no_engine_ms = engine_in_graph_ms(model, one_step, max(5, min(args.steps, 10)))
+        no_engine_ms = engine_in_graph_ms(model, one_step, args.steps)
         log('step without the engine: %.2f ms' % no_engine_ms)
     prof = None if args.no_roofline else engine_profile(model, batches[0])     # every rank runs the same (collective-bearing) step
     if rank == 0:
@@ -480,7 +533,12 @@ def main():
     ap.add_argument('--no-cpu', action='store_true', help='skip the cpu_baseline leg')
     ap.add_argument('--no-roofline', action='store_true', help='skip the roofline legs (gate kernels, whole-engine profile)')
     ap.add_argument('--config', default='cfg2', choices=sorted(CONFIGS), help='BASELINE.json configs[i-1]; the metric is quoted on cfg2')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write what the last timed step computed to DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs applies to --impl ours')
     select_config(args.config)
     if args.impl == 'reference':
         run_reference(args)
