@@ -60,8 +60,8 @@ int vp_version(void);
  * tf.nn.conv3d (ops.py:773) and their gradients.
  * wpacked: [kd*kh*kw][n_pad][kc*32] floats (see vp_pack_weights); GEMM N = n_pad (multiple of 16),
  * GEMM K = kc 32-channel chunks of in->c per tap.  out->c columns are stored.
- * split_k > 1: partial sums are atomically added into `out` (caller zero-fills; act must be NONE;
- * bias is added by split 0).  split_k == 0: automatic -- an under-filled grid with a long K loop is split and a DENSE
+ * split_k > 1: partial sums are atomically added into `out` (caller zero-fills, or leaves the prior of accumulate = 1 / 2
+ * in place; act must be NONE; bias is added by split 0).  split_k == 0: automatic -- an under-filled grid with a long K loop is split and a DENSE
  * output (out->c == out->cstride) is cleared by the call itself.  accumulate = 1: out += result (act must be NONE);
  * accumulate = 2: out = act(out + result + bias) -- the last pass of a multi-pass (3xTF32) accumulation. */
 int vp_conv_igemm(const vp_tensor* in, const vp_conv_geom* g, const float* wpacked, int n_pad, int kc,
@@ -73,6 +73,12 @@ int vp_conv_igemm(const vp_tensor* in, const vp_conv_geom* g, const float* wpack
  * geometry is not eligible), -1 = default (halo unless the environment says VP_HALO=0).  Both engines compute the same
  * sums (fp32 summation order differs); the host layer times both once per geometry and keeps the faster. */
 int vp_conv_set_engine(int engine);
+
+/* What the calling thread's last vp_conv_igemm / vp_conv_igemm_actgrad / vp_conv_wgrad call launched: info[0] = kernel
+ * (0 = box mode, 1 = halo mode, 2 = weight gradient by tap groups, 3 = weight gradient by rows; -1 = none yet),
+ * info[1] = the number of K splits it ran with.  Lets a caller see which path served a call (halo mode falls back to box
+ * mode on ineligible geometries, split_k = 0 chooses the splits). */
+int vp_conv_last_launch(int* info);
 
 /* Input-gradient convolution fused with the backward of the previous layer's activation:
  *   out = (conv(in) + addend) * act'(act_output),  act' evaluated from the activation OUTPUT (lrelu/relu/sigmoid/tanh);

@@ -504,3 +504,184 @@ def test_slab_lstm_gates_fwd_bwd(L, N, P, Fl):
     close(dc0, grads[1], 5e-5, 'slab gates dc_prev')
     for a, b_, nm in zip(dgs, grads[2:], ('dg1', 'db1', 'dg2', 'db2')):
         close(a, b_, 5e-5, 'slab gates ' + nm)
+
+
+# ------------------------------------------------------------------ losses, sampling and small reductions
+def _rel(a, b, scale, tol, what):
+    err = float((a.double() - b.double()).abs().max())
+    assert err <= tol * scale, '%s: max err %g (scale %g)' % (what, err, scale)
+
+
+@pytest.mark.parametrize('n', [1, 300, 4096])
+@pytest.mark.parametrize('label', [0.0, 1.0])
+@pytest.mark.parametrize('kind', ['LSGAN', 'GAN', 'SNGAN'])
+def test_gan_loss(L, kind, label, n):
+    """Value and gradient against O.gan_loss in fp64, logits up to +-90 (value and gradient finite, the softplus form), the
+    loss ACCUMULATED into out; n = 300 and 4096 exceed one block's stride."""
+    logits = rnd(n, seed=n) * 3.0
+    logits[:min(n, 4)] = torch.tensor([30.0, -30.0, 90.0, -90.0], device='cuda')[:min(n, 4)]
+    out = torch.full((1,), 0.5, device='cuda')
+    dl = torch.full((n,), float('nan'), device='cuda')
+    L.gan_loss(logits, label, n, 2.5, kind, dl, out)
+    torch.cuda.synchronize()
+    ld = logits.double().requires_grad_(True)
+    ref = O.gan_loss(ld, label, kind)
+    # gradient of the softplus form (the sigmoid cross-entropy form cancels in fp64 too: sigmoid(30) - 1)
+    (g,) = torch.autograd.grad(2.5 * O.gan_loss(ld, label, 'SNGAN' if kind == 'GAN' else kind), ld)
+    assert bool(torch.isfinite(out).all()) and bool(torch.isfinite(dl).all())
+    _rel(out - 0.5, ref.detach().reshape(1), max(1.0, abs(float(ref))), 1e-5, '%s value' % kind)
+    err = (dl.double() - g).abs()
+    assert bool((err <= 3e-5 * g.abs() + 1e-38).all()), '%s gradient: max err %g' % (kind, float(err.max()))   # per element
+
+
+@pytest.mark.parametrize('rows,nz', [(7, 8), (300, 8), (2, 1)])
+def test_kl_loss(L, rows, nz):
+    mu, lss = rnd(rows, nz, seed=1) * 2, (torch.rand(rows, nz, device='cuda') * 20 - 10)
+    lss.view(-1)[:2] = torch.tensor([10.0, -10.0], device='cuda')[:lss.numel()]
+    out = torch.full((1,), -1.25, device='cuda')
+    L.kl_loss(mu, lss, rows, nz, out)
+    torch.cuda.synchronize()
+    ref = O.kl_loss(mu.double(), lss.double())
+    terms = (1 + lss.double().abs() + mu.double() ** 2 + torch.exp(lss.double())).sum() / rows
+    _rel(out + 1.25, ref.reshape(1), float(terms), 2e-6, 'kl value')
+
+
+def test_sample_z_clips_and_writes_back(L):
+    total = 1000
+    mu, eps = rnd(total, seed=1), rnd(total, seed=2)
+    lss = rnd(total, seed=3) * 9.0                                    # a good share beyond +-10
+    lss0 = lss.clone()
+    z = torch.full((total,), float('nan'), device='cuda')
+    L.sample_z(mu, lss, eps, z, total)
+    torch.cuda.synchronize()
+    assert int((lss0.abs() > 10).sum()) > 50
+    assert torch.equal(lss, lss0.clamp(-10.0, 10.0))
+    ref = mu.double() + torch.sqrt(torch.exp(lss.double())) * eps.double()
+    err = (z.double() - ref).abs() / (mu.double().abs() + torch.sqrt(torch.exp(lss.double())) * eps.double().abs())
+    assert float(err.max()) <= 2e-6
+
+
+@pytest.mark.parametrize('dz_on', [True, False], ids=['dz', 'no_dz'])
+@pytest.mark.parametrize('kl_on', [True, False], ids=['kl', 'no_kl'])
+def test_sample_z_bwd(L, dz_on, kl_on):
+    """dmu = dz + k mu, dlss = dz eps sqrt(e^l) / 2 + k (e^l - 1) / 2, zero where lss was clipped; kl_scale / dz may be NULL."""
+    total = 777
+    mu, eps, dz = rnd(total, seed=1), rnd(total, seed=2), rnd(total, seed=3)
+    lss = rnd(total, seed=4) * 9.0
+    z = torch.zeros(total, device='cuda')
+    L.sample_z(mu, lss, eps, z, total)                                # lss now clipped, some exactly +-10
+    k = torch.tensor([0.37], device='cuda') if kl_on else None
+    dmu, dlss = torch.full_like(mu, float('nan')), torch.full_like(mu, float('nan'))
+    L.sample_z_bwd(mu, lss, eps, dz if dz_on else None, dmu, dlss, total, k)
+    torch.cuda.synchronize()
+    kv = 0.37 if kl_on else 0.0
+    d = dz.double() if dz_on else torch.zeros(total, dtype=torch.float64, device='cuda')
+    e = torch.exp(lss.double())
+    rmu = d + kv * mu.double()
+    rl = torch.where(lss.abs() < 10, d * eps.double() * 0.5 * torch.sqrt(e) + kv * 0.5 * (e - 1), torch.zeros_like(e))
+    _rel(dmu, rmu, float(rmu.abs().max()) + 1e-30, 1e-6, 'dmu')
+    sc = (d.abs() * eps.double().abs() * 0.5 * torch.sqrt(e) + kv * 0.5 * (e + 1))
+    assert float(((dlss.double() - rl).abs() / sc.clamp(min=1e-30)).max()) <= 2e-6
+    assert bool((dlss[lss.abs() >= 10] == 0).all()) and int((lss.abs() >= 10).sum()) > 50
+
+
+@pytest.mark.parametrize('two', [False, True], ids=['dy_a', 'dy_a+dy_b'])
+@pytest.mark.parametrize('act', [1, 2, 3, 4], ids=['relu', 'lrelu', 'sigmoid', 'tanh'])
+def test_act_bwd_on_strided_views(L, act, two):
+    rows, c = 301, 6
+    pre = rnd(rows, 8, seed=1)
+    y = {1: torch.relu(pre), 2: torch.where(pre > 0, pre, 0.2 * pre), 3: torch.sigmoid(pre), 4: torch.tanh(pre)}[act]
+    dya, dyb = rnd(rows, 12, seed=2), rnd(rows, 8, seed=3)
+    dx = torch.full((rows, 10), -5.5, device='cuda')
+    before = dx.clone()
+    L.act_bwd(y.data_ptr(), 8, dya.data_ptr() + 8, 12, dyb.data_ptr() if two else 0, 8, dx.data_ptr() + 4, 10, rows, c, act, 0.2)
+    torch.cuda.synchronize()
+    g = dya[:, 2:2 + c].double() + (dyb[:, :c].double() if two else 0)
+    yd = y[:, :c].double()
+    d = {1: (yd > 0).double(), 2: torch.where(yd > 0, torch.ones_like(yd), torch.full_like(yd, 0.2)), 3: yd * (1 - yd),
+         4: 1 - yd * yd}[act]
+    _rel(dx[:, 1:1 + c], g * d, 1.0, 1e-6, 'act_bwd %d' % act)
+    assert torch.equal(dx[:, :1], before[:, :1]) and torch.equal(dx[:, 1 + c:], before[:, 1 + c:])
+
+
+@pytest.mark.parametrize('n,P,c,xs,os_', [(1, 1000, 45, 48, 45), (3, 257, 32, 32, 40), (2, 77, 100, 104, 128)])
+def test_colsum_accumulates(L, n, P, c, xs, os_):
+    """out[n*out_stride + c] += scale * sum_p x: positions not a multiple of the block's 256 rows, c not a multiple of 32."""
+    x = rnd(n, P, xs, seed=1)
+    out = rnd(n, os_, seed=2)
+    before = out.clone()
+    L.colsum(x.data_ptr(), xs, out, n, P, c, scale=0.7, out_stride=os_)
+    torch.cuda.synchronize()
+    ref = before[:, :c].double() + 0.7 * x[:, :, :c].double().sum(dim=1)
+    sc = float((before[:, :c].double().abs() + 0.7 * x[:, :, :c].double().abs().sum(dim=1)).max())
+    _rel(out[:, :c], ref, sc, 2e-6, 'colsum')
+    assert torch.equal(out[:, c:], before[:, c:])
+
+
+def test_avgpool_fwd_bwd(L):
+    n, P, c, xs = 3, 300, 200, 204
+    x = rnd(n, P, xs, seed=1)
+    y = torch.full((n, c), float('nan'), device='cuda')
+    L.avgpool(x, xs, y, n, P, c)
+    dy = rnd(n, c, seed=2)
+    dx = torch.full((n, P, xs), 9.0, device='cuda')
+    L.avgpool_bwd(dy, dx, xs, n, P, c)
+    torch.cuda.synchronize()
+    _rel(y, x[:, :, :c].double().mean(dim=1), float(x[:, :, :c].abs().double().mean(dim=1).max()), 2e-6, 'avgpool')
+    _rel(dx[:, :, :c], (dy.double() / P)[:, None, :].expand(n, P, c), float(dy.abs().max()) / P, 1e-6, 'avgpool_bwd')
+    assert bool((dx[:, :, c:] == 9.0).all())
+
+
+@pytest.mark.parametrize('accumulate', [0, 1])
+def test_axpy_channels_row_mask(L, accumulate):
+    rows, c, rpm = 90, 5, 3
+    src = rnd(rows, 8, seed=1)
+    dst = rnd(rows, 12, seed=2)
+    before = dst.clone()
+    mask = (torch.arange(rows // rpm, device='cuda') % 4 == 1).int()
+    L.axpy_channels(src.data_ptr() + 4, 8, dst.data_ptr() + 12, 12, rows, c, scale=-1.5, row_mask=mask, rows_per_mask=rpm,
+                    accumulate=bool(accumulate))
+    torch.cuda.synchronize()
+    keep = (mask.repeat_interleave(rpm) == 0).double()[:, None]
+    ref = (before[:, 3:3 + c].double() if accumulate else 0) + keep * -1.5 * src[:, 1:1 + c].double()
+    _rel(dst[:, 3:3 + c], ref, 1.0, 1e-6, 'axpy')
+    assert torch.equal(dst[:, :3], before[:, :3]) and torch.equal(dst[:, 3 + c:], before[:, 3 + c:])
+
+
+def test_select_broadcast_and_copy_are_bit_exact(L):
+    n, per = 5, 36
+    sel = torch.tensor([1, 0, 0, 1, 1], dtype=torch.int32, device='cuda')
+    a, b = rnd(n, per, seed=1), rnd(n, per, seed=2)
+    out = torch.full((n, per), float('nan'), device='cuda')
+    L.select_rows(sel, a, b, out, n, per)
+    N, P, c = 3, 50, 7
+    vec = rnd(N, 10, seed=3)
+    dst = torch.full((N, P, 16), -2.0, device='cuda')
+    L.broadcast_channels(vec, 10, dst.data_ptr() + 4 * 5, 16, N, P, c)
+    src = rnd(N * P, 12, seed=4)
+    cp = torch.full((N * P, 20), -3.0, device='cuda')
+    L.copy_channels(src.data_ptr() + 4 * 2, 12, cp.data_ptr() + 4 * 9, 20, N * P, c)
+    torch.cuda.synchronize()
+    assert torch.equal(out, torch.where(sel[:, None].bool(), a, b))
+    assert torch.equal(dst[..., 5:5 + c], vec[:, None, :c].expand(N, P, c))
+    assert bool((dst[..., :5] == -2).all()) and bool((dst[..., 5 + c:] == -2).all())
+    assert torch.equal(cp[:, 9:9 + c], src[:, 2:2 + c])
+    assert bool((cp[:, :9] == -3).all()) and bool((cp[:, 9 + c:] == -3).all())
+
+
+@pytest.mark.parametrize('mode', [1, 2, 3], ids=['l2', 'l1_accumulate', 'l2_accumulate'])
+def test_pixel_loss_l2_and_accumulate(L, mode):
+    rows, C = 1001, 3
+    pred, tgt = torch.rand(rows, 4, device='cuda'), torch.rand(rows, 8, device='cuda')
+    out = torch.full((1,), 0.75, device='cuda')
+    dp = rnd(rows, 4, seed=1)
+    before = dp.clone()
+    L.pixel_loss(pred.data_ptr(), 4, tgt.data_ptr(), 8, dp.data_ptr(), 4, rows, C, mode, rows * C, 2.0, out)
+    torch.cuda.synchronize()
+    pd = pred[:, :C].double().requires_grad_(True)
+    ref = (O.l2_loss if mode & 1 else O.l1_loss)(pd, tgt[:, :C].double())
+    (g,) = torch.autograd.grad(2.0 * ref, pd)
+    _rel(out - 0.75, ref.reshape(1), 1.0, 1e-5, 'pixel loss value')
+    want = g + (before[:, :C].double() if mode & 2 else 0)
+    _rel(dp[:, :C], want, 1.0, 1e-6, 'pixel loss gradient')
+    assert torch.equal(dp[:, C:], before[:, C:])

@@ -683,7 +683,8 @@ __global__ void gan_loss_kernel(const float* __restrict__ logits, float label, i
     } else {
       // max(x, 0) - x*y + log(1 + exp(-|x|))   (tf.nn.sigmoid_cross_entropy_with_logits)
       s += fmaxf(x, 0.f) - x * label + log1pf(expf(-fabsf(x)));
-      if (dlogits) dlogits[i] = gscale * (1.f / (1.f + expf(-x)) - label) / n;
+      // sigmoid(x) - y without the cancellation of 1 - sigmoid(x) for y = 1 (confident logits keep their tiny gradient)
+      if (dlogits) dlogits[i] = gscale * (label != 0.f ? -1.f / (1.f + expf(x)) : 1.f / (1.f + expf(-x))) / n;
     }
   }
   __shared__ float scratch[32];

@@ -1139,6 +1139,16 @@ extern "C" int vp_conv_set_engine(int engine) {
   return 0;
 }
 
+// {kernel, splits} of the calling thread's last engine launch (vp_conv_last_launch)
+static thread_local int g_last_launch[2] = {-1, 0};
+static void note_launch(int kernel, int splits) { g_last_launch[0] = kernel; g_last_launch[1] = splits; }
+extern "C" int vp_conv_last_launch(int* info) {
+  if (!info) return set_error("vp_conv_last_launch: null argument");
+  info[0] = g_last_launch[0];
+  info[1] = g_last_launch[1];
+  return 0;
+}
+
 // Host side of halo mode.  Returns 0 = launched, 1 = not eligible (the caller uses box mode), -1 = error.
 static int conv_halo_try(const vp_tensor* in, const vp_conv_geom* g, const float* wpacked, int n_pad, int kc,
                          const vp_tensor* out, const float* bias, int act, float alpha, int split_k, int accumulate,
@@ -1287,8 +1297,7 @@ static int conv_halo_try(const vp_tensor* in, const vp_conv_geom* g, const float
   A.out = out->ptr;
   A.so_w = out->cstride; A.so_h = A.so_w * out->w; A.so_d = A.so_h * out->h; A.so_n = A.so_d * out->d;
   A.out_n = out->n; A.out_d = out->d; A.out_h = out->h; A.out_w = out->w; A.out_c = out->c;
-  A.bias = bias; A.act = act; A.alpha = alpha; A.accumulate = (A.splits > 1) ? 0 : accumulate;
-  if (A.splits > 1 && accumulate == 2) return 1;
+  A.bias = bias; A.act = act; A.alpha = alpha; A.accumulate = (A.splits > 1) ? 0 : accumulate;   // as in box mode
   {
     EncodeTiledFn enc = get_encode();
     if (!enc) return set_error("cuTensorMapEncodeTiled entry point not found");
@@ -1323,6 +1332,7 @@ static int conv_halo_try(const vp_tensor* in, const vp_conv_geom* g, const float
     igemm_halo_kernel<false><<<grid, 256, std::max(smem, static_cast<size_t>(120 * 1024)), static_cast<cudaStream_t>(stream)>>>(A);
   }
   (void)mode;
+  note_launch(1, A.splits);
   return check_launch("igemm_halo_kernel");
 }
 
@@ -1398,7 +1408,9 @@ static int conv_igemm_impl(const vp_tensor* in, const vp_conv_geom* g, const flo
   A.out = out->ptr;
   A.so_w = out->cstride; A.so_h = A.so_w * out->w; A.so_d = A.so_h * out->h; A.so_n = A.so_d * out->d;
   A.out_n = out->n; A.out_d = out->d; A.out_h = out->h; A.out_w = out->w; A.out_c = out->c;
-  A.bias = bias; A.act = act; A.alpha = alpha; A.accumulate = accumulate;
+  // split over K, the partial sums are added atomically to the output as it stands: that already accumulates (accumulate
+  // 1 and 2 are the same with act NONE), and reading the prior back in every split would add it `splits` times
+  A.bias = bias; A.act = act; A.alpha = alpha; A.accumulate = A.splits > 1 ? 0 : accumulate;
   if (accumulate == 1 && act != VP_ACT_NONE) return set_error("vp_conv_igemm: accumulate = 1 needs act NONE");
   // weights: 2-D [slots*n_pad rows][kc*32]
   {
@@ -1451,6 +1463,7 @@ static int conv_igemm_impl(const vp_tensor* in, const vp_conv_geom* g, const flo
   dim3 grid(gx, n_pad / A.bn_tile, A.num_phases * A.splits);
   kernel<<<grid, 224, smem, static_cast<cudaStream_t>(stream)>>>(A);
   count_launch(1);
+  note_launch(0, A.splits);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return set_error("igemm_fwd_kernel launch failed: %s", cudaGetErrorString(e));
   return 0;
@@ -1544,6 +1557,7 @@ extern "C" int vp_conv_wgrad(const vp_tensor* x, const vp_tensor* dy, const vp_c
           dim3 grid(A.m_tiles * A.n_tiles, groups, A.splits);
           row_kernel<<<grid, 192, smem, static_cast<cudaStream_t>(stream)>>>(A);
           count_launch(1);
+          note_launch(3, A.splits);
           cudaError_t e = cudaGetLastError();
           if (e != cudaSuccess) return set_error("igemm_wgrad_row_kernel launch failed: %s", cudaGetErrorString(e));
           return 0;
@@ -1580,6 +1594,7 @@ extern "C" int vp_conv_wgrad(const vp_tensor* x, const vp_tensor* dy, const vp_c
   dim3 grid(A.m_tiles * A.n_tiles, groups, A.splits);
   igemm_wgrad_kernel<<<grid, 192, smem, static_cast<cudaStream_t>(stream)>>>(A);
   count_launch(1);
+  note_launch(2, A.splits);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return set_error("igemm_wgrad_kernel launch failed: %s", cudaGetErrorString(e));
   return 0;

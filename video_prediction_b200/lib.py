@@ -224,6 +224,16 @@ def conv_igemm_actgrad(x_view, g, wpacked, n_pad, kc, out_view, act_output_addr,
         check(lib().vp_conv_set_engine(-1))
 
 
+KERNEL_BOX, KERNEL_HALO, KERNEL_WGRAD_TAPS, KERNEL_WGRAD_ROWS = range(4)
+
+
+def last_launch():
+    """(kernel, splits) of this thread's last engine launch: kernel is one of the KERNEL_* codes (-1 before any launch)."""
+    info = (C.c_int * 2)()
+    check(lib().vp_conv_last_launch(info))
+    return info[0], info[1]
+
+
 def tf32_residual(x):
     """x - tf32_truncate(x) with the layout of x (the 'lo' operand of the fp32-exact 3xTF32 mode)."""
     assert x.is_contiguous() and x.dtype == torch.float32
